@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this engine (CUDA, through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm (oracle), host cores
+  python bench.py ... --dump-outputs DIR                    # + the last timed step's result as DIR/*.npy (same inputs every run)
 
 One "step" = one generate_event_proof over the synthetic tipset of BASELINE.json configs[3]
 (1 M receipts x 8 events, 0.1 % match rate, events-AMT bit widths 3/5): message-AMT walk + execution
@@ -155,6 +156,44 @@ def digest_proofs(res):
     return h.hexdigest()
 
 
+# row caps of --dump-outputs: at these caps the files come to 57 MB in all, under the 64 MB a dump may take
+DUMP_CAPS = {"matching": 1 << 19, "proofs": 1 << 16, "witness": 200_000, "bytes": 1 << 20}
+
+
+def dump_outputs(res, out_dir):
+    """Writes one generate_event_proof result (EventResultPy) to out_dir/<name>.npy as float64 (integers below 2**53, exact) or
+    float32 (bytes, exact), so that two builds can be compared output for output. A table longer than its cap in DUMP_CAPS keeps
+    the rows a fixed-seed generator picks; `counts` holds the full sizes."""
+    def rows(name, n):
+        if n <= DUMP_CAPS[name]:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(20261017).choice(n, DUMP_CAPS[name], replace=False))
+
+    w = res.witness
+    blocks = np.frombuffer(b"".join(w.blocks()), dtype=np.uint8)
+    proofs = [res.proofs[i] for i in rows("proofs", len(res.proofs))]
+    payload = np.frombuffer(b"".join(b"".join(p.topics) + p.data for p in proofs), dtype=np.uint8)
+    wi = rows("witness", w.n_blocks)
+    out = {
+        "counts": np.array([len(res.matching), len(res.proofs), res.n_exec, w.n_blocks, len(blocks)], dtype=np.float64),
+        "matching": res.matching[rows("matching", len(res.matching))].astype(np.float64),
+        # per proof: exec_index, event_index, emitter, number of topics, data length
+        "proof_fields": np.array([(p.exec_index, p.event_index, p.emitter, len(p.topics), len(p.data)) for p in proofs],
+                                 dtype=np.float64).reshape(-1, 5),
+        "proof_message_cids": np.frombuffer(b"".join(p.message_cid for p in proofs), dtype=np.uint8).astype(np.float32).reshape(-1, 38),
+        # every proof's topics then its data, proofs in order
+        "proof_payload": payload[rows("bytes", len(payload))].astype(np.float32),
+        "witness_cids": w.cids[wi].astype(np.float32),
+        "witness_lengths": w.lengths[wi].astype(np.float64),
+        # witness block bytes, blocks in CID order
+        "witness_bytes": blocks[rows("bytes", len(blocks))].astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"wrote {len(out)} arrays ({sum(a.nbytes for a in out.values()) / 1e6:.1f} MB) to {out_dir}")
+
+
 # ------------------------------------------------------------------------------------------ reference arm
 def run_reference(args, world, rank):
     if rank != 0:
@@ -168,21 +207,27 @@ def run_reference(args, world, rank):
     d, keep = A.make_tipset_desc(ts)
     L = oracle.lib()
 
-    def step():
+    def step(hold=False):
+        """hold: also return the result unfreed (the caller frees it)."""
         out = C.POINTER(A.EventResultC)()
         rc = L.oracle_generate_event_proof(st._h, C.byref(d), C.byref(spec), 0, cores, C.byref(out))
         assert rc == 0, L.oracle_last_error()
         r = out.contents
         res = (int(r.n_matching), int(r.witness.n_blocks), int(r.witness.blob_size), int(r.n_proofs), int(r.n_exec))
+        if hold:
+            return res, out
         L.oracle_event_result_free(out)
-        return res
+        return res, None
 
     for _ in range(max(args.warmup, 1)):
         step()
     t0 = time.time()
-    for _ in range(args.steps):
-        nm, wb, wbytes, npf, nex = step()
+    for i in range(args.steps):
+        (nm, wb, wbytes, npf, nex), last = step(hold=args.dump_outputs is not None and i == args.steps - 1)
     dt = time.time() - t0
+    if last is not None:
+        dump_outputs(A.event_result_from_c(last.contents), args.dump_outputs)
+        L.oracle_event_result_free(last)
     val = ts.n_receipts * args.steps / dt
     line = {
         "impl": "reference", "metric": "receipts/sec scanned", "value": val, "unit": "receipts/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -325,7 +370,8 @@ def run_engine(args, world, rank, local):
 
     stats = {}
 
-    def step_resident(full=True):
+    def step_resident(full=True, hold=False):
+        """hold: return the result unfreed (the caller frees it) instead of freeing it here."""
         out = run_shard(store, tip)
         r = out.contents
         m = int(r.witness.n_blocks)
@@ -340,6 +386,8 @@ def run_engine(args, world, rank, local):
                      pass1_bytes=int(r.pass1_bytes), pass1_nodes=int(r.pass1_nodes),
                      d2h_bytes=int(r.n_matching) * 4 + int(r.n_proofs) * C.sizeof(A.EventProofC) + int(r.data_blob_size) +
                      int(r.witness.n_blocks) * (38 + 8 + 4) + int(r.witness.blob_size))
+        if hold:
+            return out
         L.ipcfp_event_result_free(out)
 
     def barrier():
@@ -366,15 +414,20 @@ def run_engine(args, world, rank, local):
     t_wall0 = time.time()
     ev0.record(ext_stream)
     step_wall = []
-    for _ in range(args.steps):
+    for i in range(args.steps):
         _t = time.perf_counter()
-        step_resident(False)
+        # --dump-outputs: the last timed step's result stays alive until after the timed region
+        last = step_resident(False, hold=args.dump_outputs is not None and i == args.steps - 1)
         step_wall.append(1e3 * (time.perf_counter() - _t))
         for k in phase:
             phase[k].append(stats["ms"][k])
     ev1.record(ext_stream)
     torch.cuda.synchronize()
     t_wall1 = time.time()
+    if last is not None:
+        if rank == 0:
+            dump_outputs(A.event_result_from_c(last.contents), args.dump_outputs)
+        L.ipcfp_event_result_free(last)
     barrier()
     launches = api.kernel_launch_count() - launches0
     # CUDA events on the engine stream bracket the K steps on every rank (each step ends with the results on the host); max over ranks
@@ -575,7 +628,11 @@ def main():
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-storage", action="store_true", help="skip the HAMT storage-lookup section (configs[2])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (rank 0; "
+                                                           "float32 / float64, under 64 MB, large tables sampled at fixed-seed rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world, rank, local = dist_env()
     if args.impl == "reference":
         run_reference(args, world, rank)

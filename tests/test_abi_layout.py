@@ -6,6 +6,9 @@ import re
 import subprocess
 import tempfile
 
+import numpy as np
+import pytest
+
 from ipc_filecoin_proofs_b200 import _abi as A
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -61,6 +64,51 @@ def test_bench_reference_arm_contract():
         assert k in d, k
     assert d["impl"] == "reference" and d["unit"] == "receipts/s" and d["value"] > 0
     assert d["cpu_baseline"]["kind"] == "port" and d["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def _bench_dump(out_dir, *argv):
+    """bench.py on a 3000-receipt tipset with `--dump-outputs out_dir` → (its JSON line, {name: array} of what it wrote)."""
+    import json
+    import sys
+    env = dict(os.environ, IPCFP_BENCH_RECEIPTS="3000")
+    out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), *argv, "--dump-outputs", str(out_dir)], env=env, text=True,
+                                  stderr=subprocess.DEVNULL)
+    return json.loads(out), {f[:-len(".npy")]: np.load(os.path.join(out_dir, f)) for f in os.listdir(out_dir)}
+
+
+def test_bench_dump_outputs_reference_arm(tmp_path, synth_mod, oracle_mod):
+    """`bench.py --dump-outputs DIR` writes the last timed step's result as float32 / float64 arrays; the same arguments give the same
+    inputs, so two runs (of different --steps) write the same arrays, and they are the oracle's result on the benchmark's tipset."""
+    (la, a), (lb, b) = [_bench_dump(tmp_path / str(k), "--impl", "reference", "--steps", str(k), "--warmup", "0") for k in (1, 2)]
+    assert (la["steps"], lb["steps"]) == (1, 2)
+    assert sorted(a) == sorted(b) == ["counts", "matching", "proof_fields", "proof_message_cids", "proof_payload", "witness_bytes",
+                                      "witness_cids", "witness_lengths"]
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k]), k
+    ts = synth_mod.Tipset(synth_mod.config_params(4, n_receipts=3000))
+    exp = oracle_mod.Store.from_tipset(ts).generate_event_proof(ts, A.make_event_spec(ts.event_signature, ts.topic1, ts.actor_filter))
+    blocks = b"".join(exp.witness.blocks())
+    assert a["counts"].tolist() == [len(exp.matching), len(exp.proofs), exp.n_exec, exp.witness.n_blocks, len(blocks)]
+    assert len(exp.proofs) > 0 and exp.witness.n_blocks > 0
+    assert np.array_equal(a["matching"], exp.matching) and np.array_equal(a["witness_cids"], exp.witness.cids)
+    assert np.array_equal(a["witness_lengths"], exp.witness.lengths) and np.array_equal(a["witness_bytes"], np.frombuffer(blocks, np.uint8))
+    assert a["proof_fields"][:, 0].tolist() == [p.exec_index for p in exp.proofs]
+    assert np.array_equal(a["proof_message_cids"], np.array([list(p.message_cid) for p in exp.proofs]))
+    assert np.array_equal(a["proof_payload"], np.frombuffer(b"".join(b"".join(p.topics) + p.data for p in exp.proofs), np.uint8))
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_engine_equals_reference_arm(tmp_path):
+    """The engine arm's dump equals the reference arm's array for array on the same inputs, and --steps sets the number of timed
+    steps: the kernel launches counted over the timed region grow with it."""
+    _, ref = _bench_dump(tmp_path / "ref", "--impl", "reference", "--steps", "1", "--warmup", "0")
+    (l2, g2), (l3, g3) = [_bench_dump(tmp_path / str(k), "--steps", str(k), "--warmup", "1", "--no-storage", "--no-cpu-baseline") for k in (2, 3)]
+    for got in (g2, g3):
+        assert sorted(got) == sorted(ref)
+        for k in ref:
+            assert np.array_equal(got[k], ref[k]), k
+    assert (l2["steps"], l3["steps"]) == (2, 3)
+    assert l3["gpu_launches"] > l2["gpu_launches"] > 0
 
 
 def test_rust_shim_uses_only_declared_bindings():
