@@ -256,6 +256,25 @@ ipcfp_status ipcfp_generate_event_proof(ipcfp_store* s, const ipcfp_tipset_desc*
                                         uint32_t flags, ipcfp_event_result** out);
 void ipcfp_event_result_free(ipcfp_event_result* r);
 
+/* The event half of generate_proof_bundle (src/proofs/generator.rs:57-78) in ONE scan of the tipset for n_specs specs
+ * (1 ≤ n_specs ≤ IPCFP_MAX_EVENT_SPECS): base witness, message-AMT walk and execution order once, one pass-1 launch that tests every
+ * spec on every StampedEvent, pass 2 over the union of the specs' matches, and ONE witness: the BTreeSet union of the specs'
+ * witnesses. With B = ipcfp_generate_proof_bundle(s, t, NULL, 0, specs, n_specs):
+ *   matching_indices  the concatenation in spec order of B.events[k].matching_indices; spec k's part is
+ *                     [spec_match_offsets[k], spec_match_offsets[k+1]), n_matching the total
+ *   proofs            the concatenation in spec order of B.events[k].proofs; spec k's part is [spec_proof_offsets[k], spec_proof_offsets[k+1])
+ *   data_blob         the concatenation in spec order of the specs' data blobs; topics_off / data_off point into it
+ *   witness, n_exec   B.witness byte for byte; the single call's n_exec
+ * Identical specs give their proofs twice; a spec that matches nothing has an empty part. Flags as for ipcfp_generate_event_proof
+ * (IPCFP_WITNESS_BY_REFERENCE, IPCFP_SCAN_SKIP_TX_AMTS); the sharded flags give IPCFP_ERR_INVALID_ARG. A failure is the one B
+ * reports: setup, message-AMT walk and pass-1 faults, then spec 0's pass-2 faults, spec 0's missing base-witness block, spec 1's
+ * pass-2 faults, and so on. The offset arrays (n_specs + 1 entries each) belong to the caller. The result is an ordinary
+ * ipcfp_event_result for ipcfp_event_result_free, ipcfp_event_result_to_json and ipcfp_verify_event_proofs. */
+#define IPCFP_MAX_EVENT_SPECS 64
+ipcfp_status ipcfp_generate_event_proof_multi(ipcfp_store* s, const ipcfp_tipset_desc* t, const ipcfp_event_spec* specs, uint32_t n_specs,
+                                              uint32_t flags, uint64_t* spec_match_offsets, uint64_t* spec_proof_offsets,
+                                              ipcfp_event_result** out);
+
 /* Device-resident tipset descriptor: upload once, scan many specs against it (the reference calls
  * generate_event_proof once per EventProofSpec with the same tipsets, proofs/generator.rs:58-78). */
 typedef struct ipcfp_tipset ipcfp_tipset;
@@ -265,6 +284,10 @@ ipcfp_status ipcfp_generate_event_proof_resident(ipcfp_store* s, ipcfp_tipset* t
                                                  ipcfp_event_result** out);
 ipcfp_status ipcfp_generate_event_proof_shard_resident(ipcfp_store* s, ipcfp_tipset* t, const ipcfp_event_spec* spec, uint64_t lo,
                                                        uint64_t hi, uint32_t world_size, uint32_t rank, uint32_t flags,
+                                                       ipcfp_event_result** out);
+/* ipcfp_generate_event_proof_multi against a device-resident tipset */
+ipcfp_status ipcfp_generate_event_proof_multi_resident(ipcfp_store* s, ipcfp_tipset* t, const ipcfp_event_spec* specs, uint32_t n_specs,
+                                                       uint32_t flags, uint64_t* spec_match_offsets, uint64_t* spec_proof_offsets,
                                                        ipcfp_event_result** out);
 /* The CUDA stream (cudaStream_t) all work of this store is issued on — for callers that time with
  * CUDA events or order their own device work after the engine's. */

@@ -24,6 +24,7 @@ pub const IPCFP_SHARDED_UNION_TO_HOST: u32 = 0x2;
 pub const IPCFP_SHARDED_UNION_FULL: u32 = 0x4;
 pub const IPCFP_WITNESS_BY_REFERENCE: u32 = 0x8;
 pub const IPCFP_COMM_ID_BYTES: usize = 128;
+pub const IPCFP_MAX_EVENT_SPECS: u32 = 64;
 
 #[repr(C)] pub struct ipcfp_store { _p: [u8; 0] }
 #[repr(C)] pub struct ipcfp_tipset { _p: [u8; 0] }
@@ -110,6 +111,12 @@ extern "C" {
     pub fn ipcfp_generate_event_proof(s: *mut ipcfp_store, t: *const ipcfp_tipset_desc, spec: *const ipcfp_event_spec, flags: u32,
                                       out: *mut *mut ipcfp_event_result) -> ipcfp_status;
     pub fn ipcfp_event_result_free(r: *mut ipcfp_event_result);
+    pub fn ipcfp_generate_event_proof_multi(s: *mut ipcfp_store, t: *const ipcfp_tipset_desc, specs: *const ipcfp_event_spec, n_specs: u32, flags: u32,
+                                            spec_match_offsets: *mut u64, spec_proof_offsets: *mut u64,
+                                            out: *mut *mut ipcfp_event_result) -> ipcfp_status;
+    pub fn ipcfp_generate_event_proof_multi_resident(s: *mut ipcfp_store, t: *mut ipcfp_tipset, specs: *const ipcfp_event_spec, n_specs: u32, flags: u32,
+                                                     spec_match_offsets: *mut u64, spec_proof_offsets: *mut u64,
+                                                     out: *mut *mut ipcfp_event_result) -> ipcfp_status;
     pub fn ipcfp_tipset_upload(s: *mut ipcfp_store, t: *const ipcfp_tipset_desc, out: *mut *mut ipcfp_tipset) -> ipcfp_status;
     pub fn ipcfp_tipset_free(t: *mut ipcfp_tipset);
     pub fn ipcfp_generate_event_proof_resident(s: *mut ipcfp_store, t: *mut ipcfp_tipset, spec: *const ipcfp_event_spec, flags: u32,

@@ -43,7 +43,7 @@ EXPORTS = [
     "ipcfp_store_stream", "ipcfp_exec_bucketize", "ipcfp_exec_dedup", "ipcfp_exec_fetch",
     "ipcfp_comm_unique_id", "ipcfp_comm_init", "ipcfp_comm_destroy", "ipcfp_generate_event_proof_sharded",
     "ipcfp_verify_event_proofs", "ipcfp_verify_storage_proofs", "ipcfp_bundle_to_json", "ipcfp_event_result_to_json", "ipcfp_json_free",
-    "ipcfp_bundle_from_json", "ipcfp_parsed_bundle_free",
+    "ipcfp_bundle_from_json", "ipcfp_parsed_bundle_free", "ipcfp_generate_event_proof_multi", "ipcfp_generate_event_proof_multi_resident",
 ]
 
 
@@ -86,6 +86,12 @@ def lib():
         L.ipcfp_generate_event_proof_shard.argtypes = [C.c_void_p, C.POINTER(A.TipsetDesc), C.POINTER(A.EventSpec), C.c_uint64, C.c_uint64,
                                                        C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(C.POINTER(A.EventResultC))]
         L.ipcfp_event_result_free.argtypes = [C.POINTER(A.EventResultC)]
+        L.ipcfp_generate_event_proof_multi.restype = C.c_int32
+        L.ipcfp_generate_event_proof_multi.argtypes = [C.c_void_p, C.POINTER(A.TipsetDesc), C.POINTER(A.EventSpec), C.c_uint32, C.c_uint32,
+                                                       C.c_void_p, C.c_void_p, C.POINTER(C.POINTER(A.EventResultC))]
+        L.ipcfp_generate_event_proof_multi_resident.restype = C.c_int32
+        L.ipcfp_generate_event_proof_multi_resident.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(A.EventSpec), C.c_uint32, C.c_uint32,
+                                                                C.c_void_p, C.c_void_p, C.POINTER(C.POINTER(A.EventResultC))]
         L.ipcfp_read_storage_slots.restype = C.c_int32
         L.ipcfp_read_storage_slots.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.POINTER(A.SlotResultC))]
         L.ipcfp_slot_result_free.argtypes = [C.POINTER(A.SlotResultC)]
@@ -175,6 +181,21 @@ class StorageProofSpec:  # reference src/proofs/generator.rs:12-15
     slot: bytes
 
 
+@dataclass
+class MultiEventResult:
+    """Result of BlockStore.generate_event_proof_multi: one EventResultPy for all specs (witness = the union of the specs'
+    witnesses), with spec k's matching receipts at match_offsets[k]:match_offsets[k+1] and its proofs at
+    proof_offsets[k]:proof_offsets[k+1]."""
+    result: A.EventResultPy
+    match_offsets: np.ndarray
+    proof_offsets: np.ndarray
+
+    def spec(self, k):
+        """(matching receipt indices, proofs) of spec k."""
+        m, p = self.match_offsets, self.proof_offsets
+        return self.result.matching[int(m[k]):int(m[k + 1])], self.result.proofs[int(p[k]):int(p[k + 1])]
+
+
 class PinnedArray:
     """Pinned host memory (ipcfp_host_alloc) exposed as a numpy array."""
 
@@ -254,6 +275,30 @@ class BlockStore:
         finally:
             lib().ipcfp_event_result_free(out)
 
+    # --- the event specs of generate_proof_bundle (proofs/generator.rs:57-78) in one scan of the tipset
+    def generate_event_proof_multi(self, ts, specs, flags=0):
+        d, keep = A.make_tipset_desc(ts)
+        return self._multi(lambda *a: lib().ipcfp_generate_event_proof_multi(self._h, C.byref(d), *a), specs, flags)
+
+    def generate_event_proof_multi_resident(self, tipset, specs, flags=0):
+        """The same against a ResidentTipset of this store."""
+        return self._multi(lambda *a: lib().ipcfp_generate_event_proof_multi_resident(self._h, tipset._h, *a), specs, flags)
+
+    def upload_tipset(self, ts):
+        return ResidentTipset(self, ts)
+
+    @staticmethod
+    def _multi(call, specs, flags):
+        cs = [s.as_c() if isinstance(s, EventProofSpec) else s for s in specs]
+        arr = (A.EventSpec * max(len(cs), 1))(*cs)
+        mo, po = np.zeros(len(cs) + 1, dtype=np.uint64), np.zeros(len(cs) + 1, dtype=np.uint64)
+        out = C.POINTER(A.EventResultC)()
+        _check(call(arr, len(cs), flags, mo.ctypes.data, po.ctypes.data, C.byref(out)))
+        try:
+            return MultiEventResult(A.event_result_from_c(out.contents), mo, po)
+        finally:
+            lib().ipcfp_event_result_free(out)
+
     def generate_event_proof_shard(self, ts, spec, lo, hi, world, rank, flags=0):
         d, keep = A.make_tipset_desc(ts)
         cs = spec.as_c() if isinstance(spec, EventProofSpec) else spec
@@ -304,6 +349,26 @@ class BlockStore:
     def close(self):
         if self._h:
             lib().ipcfp_store_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class ResidentTipset:
+    """A tipset descriptor uploaded to the device once (ipcfp_tipset_upload) for many calls against one BlockStore."""
+
+    def __init__(self, store, ts):
+        d, keep = A.make_tipset_desc(ts)
+        self._h = C.c_void_p()
+        _check(lib().ipcfp_tipset_upload(store._h, C.byref(d), C.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            lib().ipcfp_tipset_free(self._h)
             self._h = None
 
     def __del__(self):

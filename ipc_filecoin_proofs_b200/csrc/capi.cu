@@ -209,6 +209,20 @@ ipcfp_status ipcfp_generate_event_proof_shard(ipcfp_store* s, const ipcfp_tipset
     });
 }
 void ipcfp_event_result_free(ipcfp_event_result* r) { if (r) event_result_free(r); }
+ipcfp_status ipcfp_generate_event_proof_multi(ipcfp_store* s, const ipcfp_tipset_desc* t, const ipcfp_event_spec* specs, uint32_t n_specs, uint32_t flags,
+                                              uint64_t* spec_match_offsets, uint64_t* spec_proof_offsets, ipcfp_event_result** out) {
+    return guard([&] {
+        if (!s || !out) throw Error(IPCFP_ERR_INVALID_ARG, "null argument");
+        *out = nullptr;
+        Store* st = reinterpret_cast<Store*>(s);
+        const MultiSpecs ms{specs, n_specs, spec_match_offsets, spec_proof_offsets};
+        if (!specs || !spec_match_offsets || !spec_proof_offsets) throw Error(IPCFP_ERR_INVALID_ARG, "null argument");
+        if (n_specs == 0 || n_specs > IPCFP_MAX_EVENT_SPECS) throw Error(IPCFP_ERR_INVALID_ARG, "n_specs must be 1..IPCFP_MAX_EVENT_SPECS");
+        TipsetDev td;
+        tipset_upload(st, t, td);
+        *out = generate_event_proof(st, t, td, nullptr, flags, false, 0, 0, 1, 0, nullptr, nullptr, &ms);
+    });
+}
 
 ipcfp_status ipcfp_tipset_upload(ipcfp_store* s, const ipcfp_tipset_desc* t, ipcfp_tipset** out) {
     return guard([&] {
@@ -228,6 +242,16 @@ ipcfp_status ipcfp_generate_event_proof_resident(ipcfp_store* s, ipcfp_tipset* t
         if (!s || !t || !out) throw Error(IPCFP_ERR_INVALID_ARG, "null argument");
         *out = nullptr;
         *out = generate_event_proof(reinterpret_cast<Store*>(s), nullptr, *reinterpret_cast<TipsetDev*>(t), spec, flags, false, 0, 0, 1, 0);
+    });
+}
+ipcfp_status ipcfp_generate_event_proof_multi_resident(ipcfp_store* s, ipcfp_tipset* t, const ipcfp_event_spec* specs, uint32_t n_specs, uint32_t flags,
+                                                       uint64_t* spec_match_offsets, uint64_t* spec_proof_offsets, ipcfp_event_result** out) {
+    return guard([&] {
+        if (!s || !t || !out) throw Error(IPCFP_ERR_INVALID_ARG, "null argument");
+        *out = nullptr;
+        const MultiSpecs ms{specs, n_specs, spec_match_offsets, spec_proof_offsets};
+        *out = generate_event_proof(reinterpret_cast<Store*>(s), nullptr, *reinterpret_cast<TipsetDev*>(t), nullptr, flags, false, 0, 0, 1, 0, nullptr,
+                                    nullptr, &ms);
     });
 }
 ipcfp_status ipcfp_generate_event_proof_shard_resident(ipcfp_store* s, ipcfp_tipset* t, const ipcfp_event_spec* spec, uint64_t lo, uint64_t hi,

@@ -116,9 +116,16 @@ struct ExecOrderOut {
     AsyncBuf<RawCid> exec_raw;
     AsyncBuf<uint32_t> exec_idx;
 };
+// ipcfp_generate_event_proof_multi: n specs scanned together; the caller's offset arrays have n + 1 entries each
+struct MultiSpecs {
+    const ipcfp_event_spec* specs;
+    uint32_t n;
+    uint64_t* match_off;
+    uint64_t* proof_off;
+};
 ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* t, TipsetDev& td, const ipcfp_event_spec* spec, uint32_t flags,
                                          bool sharded, uint64_t lo, uint64_t hi, uint32_t world, uint32_t rank, Comm* comm = nullptr,
-                                         ExecOrderOut* exo = nullptr);
+                                         ExecOrderOut* exo = nullptr, const MultiSpecs* ms = nullptr);
 // verify.cu — batched verifiers over a witness store
 void verify_event_proofs(Store* s, const ipcfp_tipset_desc* t, const ipcfp_event_proof* proofs, uint64_t n, const uint8_t* data_blob, uint64_t blob_size,
                          const ipcfp_event_spec* filter, uint8_t* results);

@@ -170,6 +170,86 @@ __global__ void __launch_bounds__(128) k_pass2(Pass2Args a) {
     pass2_item(a, t);
 }
 
+// ------------------------------------------------------------------------------------------ several specs in one scan (per-item code: events_items.cuh)
+// keccak256(event_signature) → m[k].t0 for every spec, one thread per spec (k_setup's thread 96 does it for one)
+__global__ void k_spec_keccak(MultiMatcher* mm, const uint8_t* sigs, const uint32_t* sig_off, const uint32_t* sig_len) {
+    const uint32_t k = threadIdx.x;
+    if (k >= mm->n) return;
+    Digest d;
+    keccak256(sigs + sig_off[k], sig_len[k], d);
+    for (int w = 0; w < 4; w++) mm->m[k].t0[w] = d.w[w];
+}
+// k_pass1_occ8's thread-per-root shape with every spec tested on every event. The specs are staged in shared memory: the screen of
+// event_spec_mask reads two words per spec and event. The ballot gives the bitmap of receipts some spec matches.
+__global__ void __launch_bounds__(128, 8) k_pass1_multi(Pass1MultiArgs a) {
+    __shared__ MultiMatcher s_mm;
+    const uint32_t n_specs = a.mm->n;
+    for (uint32_t w = threadIdx.x; w < n_specs * (uint32_t)(sizeof(Matcher) / 8); w += blockDim.x) ((uint64_t*)s_mm.m)[w] = ((const uint64_t*)a.mm->m)[w];
+    if (threadIdx.x == 0) s_mm.n = n_specs;
+    __syncthreads();
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int32_t blk = pass1_multi_lookup(a, i);
+    uint32_t len = 0, bytes = 0, nodes = 0;
+    const uint8_t* p = nullptr;
+    if (blk >= 0) {
+        p = store_block(a.store, (uint32_t)blk, len);
+        for (uint32_t o = 0; o < len && o < 512; o += 128) prefetch_l2(p + o);
+    }
+    __syncwarp();
+    uint64_t mask = 0;
+    WalkOut wo{0, 0, false};
+    if (blk >= 0) {
+        bytes = len + 38; nodes = 1;
+        mask = pass1_multi_decode(a, s_mm, i, (uint32_t)blk, p, len, wo);
+    }
+    if (mask) a.spec_mask[i] = mask;
+    const unsigned b = __ballot_sync(0xffffffffu, mask != 0);
+    if ((threadIdx.x & 31) == 0) a.match_bits[i >> 5] = b;
+    uint32_t pairs = (uint32_t)__popcll(mask), np_ = wo.nproofs, nb_ = wo.nbytes;
+    for (int o = 16; o; o >>= 1) {
+        bytes += __shfl_xor_sync(0xffffffffu, bytes, o); nodes += __shfl_xor_sync(0xffffffffu, nodes, o);
+        pairs += __shfl_xor_sync(0xffffffffu, pairs, o); np_ += __shfl_xor_sync(0xffffffffu, np_, o); nb_ += __shfl_xor_sync(0xffffffffu, nb_, o);
+    }
+    if ((threadIdx.x & 31) == 0 && nodes) { atomicAdd(a.stats, (unsigned long long)nodes); atomicAdd(a.stats + 1, (unsigned long long)bytes); }
+    if ((threadIdx.x & 31) == 0 && pairs) {
+        atomicAdd(a.n_pairs, (unsigned long long)pairs); atomicAdd(a.n_proofs, (unsigned long long)np_); atomicAdd(a.n_bytes, (unsigned long long)nb_);
+    }
+}
+// bit k * stride + t of the pair bitmap for every spec k matching match t
+__global__ void k_pair_bits(const uint32_t* __restrict__ match_rel, const uint64_t* __restrict__ spec_mask, uint64_t n_match, uint64_t stride, uint32_t* pair_bits) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_match) return;
+    for (uint64_t m = spec_mask[match_rel[t]]; m; m &= m - 1) {
+        const uint64_t bit = (uint64_t)(__ffsll((long long)m) - 1) * stride + t;
+        atomicOr(&pair_bits[bit >> 5], 1u << (bit & 31));
+    }
+}
+__global__ void __launch_bounds__(128) k_pair_count(StoreView store, const StoreView* store_dev, const MultiMatcher* mm, const uint8_t* events_roots,
+                                                    const uint32_t* match_rel, const uint32_t* pairs, uint64_t n_pairs, uint64_t stride, uint32_t* cnt,
+                                                    uint32_t* nbytes) {
+    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_pairs) return;
+    pair_count_item(store, store_dev, mm, events_roots, match_rel, pairs, stride, q, cnt, nbytes);
+}
+// per spec k = 0..n_specs: its first pair, proof and blob byte in the spec-major layout (out[k], out[n+1+k], out[2(n+1)+k])
+__global__ void k_spec_bounds(const uint32_t* __restrict__ pairs, uint64_t n_pairs, uint64_t stride, const uint64_t* __restrict__ pbase,
+                              const uint64_t* __restrict__ bbase, uint64_t n_proofs, uint64_t n_bytes, uint32_t n_specs, uint64_t* out) {
+    const uint32_t k = threadIdx.x;
+    if (k > n_specs) return;
+    uint64_t lo = 0, hi = n_pairs;
+    while (lo < hi) { const uint64_t mid = (lo + hi) / 2; if (pairs[mid] < k * stride) lo = mid + 1; else hi = mid; }
+    out[k] = lo;
+    out[n_specs + 1 + k] = lo < n_pairs ? pbase[lo] : n_proofs;
+    out[2 * (n_specs + 1) + k] = lo < n_pairs ? bbase[lo] : n_bytes;
+}
+// one matching receipt per warp up to 16 384 matches, one per thread above (k_pass2's shapes)
+__global__ void __launch_bounds__(128) k_pass2_multi(Pass2MultiArgs a) {
+    uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (a.per_warp) { if (threadIdx.x & 31) return; t >>= 5; }
+    if (t >= a.n_match) return;
+    pass2_multi_item(a, t);
+}
+
 // ------------------------------------------------------------------------------------------ setup + message AMT walk
 #define IPCFP_MAX_PARENTS 64
 struct SetupArgs {
@@ -477,11 +557,24 @@ void tipset_upload(Store* s, const ipcfp_tipset_desc* t, TipsetDev& td) {
 }
 
 ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*/, TipsetDev& td, const ipcfp_event_spec* spec, uint32_t flags,
-                                         bool sharded, uint64_t lo, uint64_t hi, uint32_t world, uint32_t rank, Comm* comm, ExecOrderOut* exo) {
+                                         bool sharded, uint64_t lo, uint64_t hi, uint32_t world, uint32_t rank, Comm* comm, ExecOrderOut* exo,
+                                         const MultiSpecs* ms) {
     s->use();
     cudaStream_t st = s->stream;
     const auto t_enter = std::chrono::steady_clock::now();
     static thread_local std::chrono::steady_clock::time_point t_last_exit = t_enter;
+    // ms: several specs in one scan (ipcfp_generate_event_proof_multi). Setup, walk, dedup and witness are the single call's; the
+    // matcher staging, pass 1, the (spec, match) counts and scans, pass 2 and the error order are its own.
+    const uint32_t K = ms ? ms->n : 1;
+    if (ms) {
+        if (!ms->specs || !ms->match_off || !ms->proof_off) throw Error(IPCFP_ERR_INVALID_ARG, "null argument");
+        if (K == 0 || K > IPCFP_MAX_EVENT_SPECS) throw Error(IPCFP_ERR_INVALID_ARG, "n_specs must be 1..IPCFP_MAX_EVENT_SPECS");
+        if (sharded || comm || exo || (flags & (IPCFP_SHARDED_UNION_TO_HOST | IPCFP_SHARDED_UNION_FULL)))
+            throw Error(IPCFP_ERR_INVALID_ARG, "the multi-spec call is not sharded");
+        for (uint32_t k = 0; k < K; k++)
+            if (!ms->specs[k].event_signature || !ms->specs[k].topic_1) throw Error(IPCFP_ERR_INVALID_ARG, "event spec has null fields");
+        spec = &ms->specs[0];
+    }
     if (!spec || !spec->event_signature || !spec->topic_1) throw Error(IPCFP_ERR_INVALID_ARG, "event spec has null fields");
     if (!sharded) { lo = 0; hi = td.n_receipts; }
     if (lo > hi || hi > td.n_receipts) throw Error(IPCFP_ERR_INVALID_ARG, "receipt range out of bounds");
@@ -516,38 +609,58 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     IPCFP_CUDA(cudaMemsetAsync(dw + 1, 0, 40 * 8, st));
     IPCFP_CUDA(cudaMemsetAsync(dw + 15, 0xff, 8, st));   // message-AMT fault word
 
-    // ---- matcher
-    Matcher mh;
-    memset(&mh, 0, sizeof mh);
-    {
-        size_t n1 = strlen(spec->topic_1);
+    // ---- matcher(s)
+    auto make_matcher = [](const ipcfp_event_spec* sp) {
+        Matcher m;
+        memset(&m, 0, sizeof m);
+        size_t n1 = strlen(sp->topic_1);
         uint8_t t1[32];
         memset(t1, 0, 32);
-        memcpy(t1, spec->topic_1, n1 < 32 ? n1 : 32);  // ascii_to_bytes32 (evm.rs:72-78)
-        memcpy(mh.t1, t1, 32);
-        mh.actor = spec->actor_id_filter;
-        mh.has_actor = spec->has_actor_id_filter ? 1 : 0;
-    }
+        memcpy(t1, sp->topic_1, n1 < 32 ? n1 : 32);  // ascii_to_bytes32 (evm.rs:72-78)
+        memcpy(m.t1, t1, 32);
+        m.actor = sp->actor_id_filter;
+        m.has_actor = sp->has_actor_id_filter ? 1 : 0;
+        return m;
+    };
+    Matcher mh = make_matcher(spec);
     // spec + tipset CIDs go up in ONE copy from the store's pinned staging block (no host sync):
     //   [0,1024) Matcher (t0 is filled in on the device) | signature, zero padded | parent, TxMeta, child, receipts-root CIDs
+    // several specs: [0, head) MultiMatcher + the signatures' offsets and lengths | the K signatures, each zero padded | CIDs
+    const size_t MULTI_SIGS = (sizeof(MultiMatcher) + 7) & ~(size_t)7;
+    const size_t head = ms ? (MULTI_SIGS + 2 * 4 * IPCFP_MAX_EVENT_SPECS + 63) & ~(size_t)63 : 1024;
+    std::vector<size_t> sig_at(K + 1, 0);
+    for (uint32_t k = 0; k < K; k++) sig_at[k + 1] = sig_at[k] + ((strlen(ms ? ms->specs[k].event_signature : spec->event_signature) + 64) & ~(size_t)63);
     const size_t siglen = strlen(spec->event_signature);
-    const size_t sig_cap = (siglen + 64) & ~(size_t)63;
+    const size_t sig_cap = sig_at[K];
     const size_t cids_bytes = 38ull * (2 * td.n_parents + 2);
-    const size_t small_bytes = 1024 + sig_cap + cids_bytes + 64;
+    const size_t small_bytes = head + sig_cap + cids_bytes + 64;
     static_assert(sizeof(Matcher) <= 1024, "Matcher must fit its staging slot");
     const size_t STAGE_TABLES = 32768;                    // second half of the staging block: dense-walk tables
     const size_t tables_off = std::max<size_t>(STAGE_TABLES, (small_bytes + 63) & ~(size_t)63);
     if (!s->stage.p || s->stage.cap < tables_off + STAGE_TABLES) s->stage = PinnedArray(s->pool, tables_off + STAGE_TABLES);
     AsyncBuf<uint8_t> small(small_bytes, st);
-    uint8_t* d_sig = small.p + 1024;                       // 8-byte aligned
-    uint8_t* d_cids = small.p + 1024 + sig_cap;
+    uint8_t* d_sig = small.p + head;                       // 8-byte aligned
+    uint8_t* d_cids = small.p + head + sig_cap;
     Matcher* d_matcher = (Matcher*)small.p;
+    MultiMatcher* d_mm = (MultiMatcher*)small.p;
     {
         uint8_t* hs = s->stage.as<uint8_t>();
         memset(hs, 0, small_bytes);
-        memcpy(hs, &mh, sizeof(Matcher));
-        memcpy(hs + 1024, spec->event_signature, siglen);
-        uint8_t* hc = hs + 1024 + sig_cap;
+        if (ms) {
+            MultiMatcher* mm = (MultiMatcher*)hs;
+            uint32_t* so = (uint32_t*)(hs + MULTI_SIGS);
+            mm->n = K;
+            for (uint32_t k = 0; k < K; k++) {
+                mm->m[k] = make_matcher(&ms->specs[k]);
+                so[k] = (uint32_t)sig_at[k];
+                so[IPCFP_MAX_EVENT_SPECS + k] = (uint32_t)strlen(ms->specs[k].event_signature);
+                memcpy(hs + head + sig_at[k], ms->specs[k].event_signature, so[IPCFP_MAX_EVENT_SPECS + k]);
+            }
+        } else {
+            memcpy(hs, &mh, sizeof(Matcher));
+            memcpy(hs + head, spec->event_signature, siglen);
+        }
+        uint8_t* hc = hs + head + sig_cap;
         memcpy(hc, td.parent_cids.data(), td.parent_cids.size()); hc += td.parent_cids.size();
         memcpy(hc, td.txmeta_cids.data(), td.txmeta_cids.size()); hc += td.txmeta_cids.size();
         memcpy(hc, td.child_cid, 38); hc += 38;
@@ -575,6 +688,10 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     sa.amt_count = amt_count.p;
     sa.sig = d_sig; sa.sig_len = (uint32_t)siglen; sa.matcher = d_matcher;
     k_setup<<<1, 256, 0, st>>>(sa); IPCFP_LAUNCH_CHECK();
+    if (ms) {
+        const uint32_t* so = (const uint32_t*)(small.p + MULTI_SIGS);
+        k_spec_keccak<<<1, IPCFP_MAX_EVENT_SPECS, 0, st>>>(d_mm, d_sig, so, so + IPCFP_MAX_EVENT_SPECS); IPCFP_LAUNCH_CHECK();
+    }
     IPCFP_CUDA(cudaMemcpyAsync(hw + 400, d_matcher, 32, cudaMemcpyDeviceToHost, st));   // t0 → hw[400..404)
     IPCFP_CUDA(cudaMemcpyAsync(hw + 24, misc.p, (64 + 2 * IPCFP_MAX_PARENTS) * 4, cudaMemcpyDeviceToHost, st));
     IPCFP_CUDA(cudaMemcpyAsync(hw + 128, amt_count.p, 2 * IPCFP_MAX_PARENTS * 8, cudaMemcpyDeviceToHost, st));
@@ -770,12 +887,21 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     }
 
     // ---- PASS 1
-    AsyncBuf<uint32_t> match_bits((N + 31) / 32 + 8, st), cnt(N + 8, st), nby(N + 8, st);
-    AsyncBuf<uint64_t> pbase(N + 8, st), bbase(N + 8, st);
+    const uint64_t N1 = ms ? 0 : N + 8;   // per-receipt counts: the single-spec pass 1 only
+    AsyncBuf<uint32_t> match_bits((N + 31) / 32 + 8, st), cnt(N1, st), nby(N1, st);
+    AsyncBuf<uint64_t> pbase(N1, st), bbase(N1, st);
     Pass1Args p1;
     p1.store = s->view; p1.store_dev = s->view_dev.p; p1.m_dev = d_matcher; p1.m = mh; p1.events_roots = td.events_roots.p; p1.has_root = td.has_root.p; p1.lo = lo; p1.hi = hi;
     p1.match_bits = match_bits.p; p1.cnt = cnt.p; p1.nbytes = nby.p; p1.err = dw; p1.stats = dw + 4;
-    if (N) {
+    AsyncBuf<uint64_t> spec_mask(ms ? N + 8 : 0, st);
+    if (ms && N) {
+        // the measured pass-1 variants (IPCFP_PASS1_*) stay on the single-spec kernel: none of them won
+        Pass1MultiArgs pm;
+        pm.store = s->view; pm.store_dev = s->view_dev.p; pm.mm = d_mm; pm.events_roots = td.events_roots.p; pm.has_root = td.has_root.p; pm.n = N;
+        pm.match_bits = match_bits.p; pm.spec_mask = spec_mask.p; pm.err = dw; pm.stats = dw + 4;
+        pm.n_proofs = dw + 7; pm.n_bytes = dw + 12; pm.n_pairs = dw + 20;
+        k_pass1_multi<<<div_up(N, 128), 128, 0, st>>>(pm); IPCFP_LAUNCH_CHECK();
+    } else if (N) {
         // kernel variant: read per call so that one process can sweep them (tools/profile_step.py)
         //   IPCFP_PASS1_STAGE=<chunk>x<slots>x<chunks per pass>   warp-cooperative shared-memory staging (pass1_stage.cuh)
         //   IPCFP_PASS1_RING=<chunk>x<slots>                      per-lane cp.async rings (pass1_ring.cuh, round-1 experiment)
@@ -820,15 +946,18 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     AsyncBuf<uint64_t> wp3((N + 31) / 32 + 8, st);
     unsigned long long* n_match_dev = dw + 6;
     bitmap_to_indices(match_bits.p, (N + 31) / 32 * 32, match_rel.p, (uint64_t*)n_match_dev, wp3.p, scratch.p, st);
-    exclusive_scan_u32(cnt.p, pbase.p, N, (uint64_t*)(dw + 7), scratch.p, st);
-    exclusive_scan_u32(nby.p, bbase.p, N, (uint64_t*)(dw + 12), scratch.p, st);
-    publish_words(s, 0, 16);
+    if (!ms) {
+        exclusive_scan_u32(cnt.p, pbase.p, N, (uint64_t*)(dw + 7), scratch.p, st);
+        exclusive_scan_u32(nby.p, bbase.p, N, (uint64_t*)(dw + 12), scratch.p, st);
+    }
+    publish_words(s, 0, ms ? 21 : 16);   // multi: proof / byte totals from pass 1 in dw[7] / dw[12], (spec, match) pairs in dw[20]
     IPCFP_CUDA(cudaStreamSynchronize(st));
     note_errors(hw);
     uint64_t n_exec = hw[3];
     const uint64_t M = hw[6];
     const uint64_t pass1_nodes = hw[4], pass1_bytes = hw[5];
     uint64_t n_proofs = hw[7], n_bytes = hw[12];
+    const uint64_t n_pairs = ms ? hw[20] : M;
 
     // ---- PASS 2
     std::unique_ptr<EventResultBox> box(new EventResultBox());
@@ -836,7 +965,32 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     AsyncBuf<ipcfp_event_proof> d_proofs(n_proofs + 1, st);
     AsyncBuf<uint8_t> d_blob(n_bytes + 16, st);
     uint32_t* any_skip_dev = misc.p + 2;
-    if (M) {
+    // multi: the (spec, match) pairs in spec-major order, their proofs and bytes, the exclusive scans, per-spec bounds
+    const uint64_t stride = (M + 31) / 32 * 32;
+    if (ms && K * stride >= 0xffffffffull) throw Error(IPCFP_ERR_UNSUPPORTED, "n_specs x matching receipts exceeds 2^32");
+    AsyncBuf<uint32_t> pair_bits(ms ? K * stride / 32 + 8 : 0, st), pairs(ms ? n_pairs + 32 : 0, st), pcnt(ms ? n_pairs + 8 : 0, st),
+        pnby(ms ? n_pairs + 8 : 0, st);
+    AsyncBuf<uint64_t> pair_prefix(ms ? K * stride / 32 + 8 : 0, st), spec_bounds(ms ? 3 * (K + 1) : 0, st);
+    if (ms && M) {
+        pbase.alloc(n_pairs + 8, st); bbase.alloc(n_pairs + 8, st);
+        AsyncBuf<uint64_t> scratch_p(scan_scratch_elems(std::max<uint64_t>(n_pairs, K * stride / 32)) + 64, st);
+        pair_bits.zero();
+        k_pair_bits<<<div_up(M, 128), 128, 0, st>>>(match_rel.p, spec_mask.p, M, stride, pair_bits.p); IPCFP_LAUNCH_CHECK();
+        // the scans below take the same launches whatever their size (≤ 16.7 M entries), so the call's launches do not depend on K
+        bitmap_to_indices(pair_bits.p, K * stride, pairs.p, (uint64_t*)(dw + 21), pair_prefix.p, scratch_p.p, st, true);
+        k_pair_count<<<div_up(n_pairs, 128), 128, 0, st>>>(s->view, s->view_dev.p, d_mm, td.events_roots.p, match_rel.p, pairs.p, n_pairs, stride, pcnt.p,
+                                                          pnby.p); IPCFP_LAUNCH_CHECK();
+        exclusive_scan_u32(pcnt.p, pbase.p, n_pairs, (uint64_t*)(dw + 22), scratch_p.p, st, true);
+        exclusive_scan_u32(pnby.p, bbase.p, n_pairs, (uint64_t*)(dw + 23), scratch_p.p, st, true);
+        k_spec_bounds<<<1, IPCFP_MAX_EVENT_SPECS + 1, 0, st>>>(pairs.p, n_pairs, stride, pbase.p, bbase.p, n_proofs, n_bytes, K, spec_bounds.p); IPCFP_LAUNCH_CHECK();
+        Pass2MultiArgs p2;
+        p2.store = s->view; p2.store_dev = s->view_dev.p; p2.mm = d_mm; p2.events_roots = td.events_roots.p; p2.match_rel = match_rel.p;
+        p2.spec_mask = spec_mask.p; p2.n_match = M; p2.receipts_root_blk = receipts_root_blk; p2.exec_cids = exec_raw.p; p2.exec_idx = exec_idx.p;
+        p2.n_exec = n_exec_dev; p2.wbits = wbits.p; p2.err = dw; p2.pair_bits = pair_bits.p; p2.pair_prefix = pair_prefix.p; p2.stride = stride;
+        p2.pair_cnt = pcnt.p; p2.proof_cur = pbase.p; p2.byte_cur = bbase.p; p2.proofs = d_proofs.p; p2.blob = d_blob.p; p2.any_skip = any_skip_dev;
+        p2.per_warp = M <= 16384 ? 1 : 0;
+        k_pass2_multi<<<div_up(p2.per_warp ? M * 32 : M, 128), 128, 0, st>>>(p2); IPCFP_LAUNCH_CHECK();
+    } else if (M) {
         Pass2Args p2;
         p2.store = s->view; p2.store_dev = s->view_dev.p; p2.m_dev = d_matcher; p2.m = mh; p2.events_roots = td.events_roots.p; p2.lo = lo; p2.match_rel = match_rel.p; p2.n_match = M;
         p2.receipts_root_blk = receipts_root_blk; p2.exec_cids = exec_raw.p; p2.exec_idx = exec_idx.p; p2.n_exec = n_exec_dev;
@@ -861,6 +1015,12 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     publish_words(s, 0, 20);
     publish_words_from(s, misc.p, 20, 2);   // misc[2] = any_skip (32-bit words 0..3 land in hw[20..21])
     IPCFP_CUDA(cudaStreamSynchronize(st));
+    if (ms && hw[0] != IPCFP_NO_ERROR && (uint32_t)(hw[0] >> 56) == ST_PASS2) {
+        // (spec, i) key of pass2_multi_item: spec 0's missing base-witness block comes after spec 0's pass-2 faults and before those of
+        // every later spec (materialize ends each of the reference's calls)
+        if ((hw[0] >> 48) & 0xff && missing_base && !skip_tx) throw Error(IPCFP_ERR_MISSING_BLOCK, "missing block (base witness CID not in the store)");
+        hw[0] &= ~(0xffull << 48);
+    }
     note_errors(hw);
     // base-witness CIDs (parent headers, child header, TxMeta) are only dereferenced by WitnessCollector::materialize
     // (common/witness.rs:43-56, events/generator.rs:104), i.e. AFTER every receipts-root / pass-1 / pass-2 failure
@@ -870,11 +1030,18 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     IPCFP_CUDA(cudaEventRecord(s->ev[4], st));
 
     // ---- results to the host
-    box->matching = PinnedArray(s->pool, (M + 1) * 8);
+    box->matching = PinnedArray(s->pool, (n_pairs + 1) * 8);
     box->proofs = PinnedArray(s->pool, (n_proofs + 1) * sizeof(ipcfp_event_proof));
     box->blob = PinnedArray(s->pool, n_bytes + 16);
     PinnedArray rel(s->pool, (M + 1) * 4);
     if (M) IPCFP_CUDA(cudaMemcpyAsync(rel.p, match_rel.p, M * 4, cudaMemcpyDeviceToHost, st));
+    PinnedArray pairs_h, bounds_h;
+    if (ms && M) {
+        pairs_h = PinnedArray(s->pool, n_pairs * 4);
+        bounds_h = PinnedArray(s->pool, 3 * (K + 1) * 8);
+        IPCFP_CUDA(cudaMemcpyAsync(pairs_h.p, pairs.p, n_pairs * 4, cudaMemcpyDeviceToHost, st));
+        IPCFP_CUDA(cudaMemcpyAsync(bounds_h.p, spec_bounds.p, 3 * (K + 1) * 8, cudaMemcpyDeviceToHost, st));
+    }
     if (n_proofs && !xch) IPCFP_CUDA(cudaMemcpyAsync(box->proofs.p, d_proofs.p, n_proofs * sizeof(ipcfp_event_proof), cudaMemcpyDeviceToHost, st));
     if (n_bytes) IPCFP_CUDA(cudaMemcpyAsync(box->blob.p, d_blob.p, n_bytes, cudaMemcpyDeviceToHost, st));
 
@@ -936,29 +1103,50 @@ ipcfp_event_result* generate_event_proof(Store* s, const ipcfp_tipset_desc* /*t*
     }
     IPCFP_CUDA(cudaEventRecord(s->ev[5], st));
     IPCFP_CUDA(cudaStreamSynchronize(st));
-    {
+    if (ms) {
+        // spec k's part of matching_indices: its pairs, in receipt order; of proofs: [proof_off[k], proof_off[k + 1])
+        uint64_t* mo = box->matching.as<uint64_t>();
+        const uint32_t* rp = rel.as<uint32_t>();
+        const uint32_t* pp = pairs_h.as<uint32_t>();
+        for (uint64_t q = 0; q < n_pairs; q++) mo[q] = rp[pp[q] % stride];
+        const uint64_t* bh = bounds_h.as<uint64_t>();
+        for (uint32_t k = 0; k <= K; k++) {
+            ms->match_off[k] = M ? bh[k] : 0;
+            ms->proof_off[k] = M ? bh[K + 1 + k] : 0;
+        }
+        if (any_skip) {   // receipts the AMT does not hold: compact every spec's part
+            ipcfp_event_proof* pr = box->proofs.as<ipcfp_event_proof>();
+            uint64_t w = 0;
+            for (uint32_t k = 0; k < K; k++) {
+                const uint64_t b = ms->proof_off[k], e = ms->proof_off[k + 1];
+                ms->proof_off[k] = w;
+                for (uint64_t j = b; j < e; j++) if (pr[j].exec_index != UINT64_MAX) pr[w++] = pr[j];
+            }
+            ms->proof_off[K] = n_proofs = w;
+        }
+    } else {
         uint64_t* mo = box->matching.as<uint64_t>();
         const uint32_t* rp = rel.as<uint32_t>();
         for (uint64_t k = 0; k < M; k++) mo[k] = lo + rp[k];
     }
-    if (any_skip) {  // receipts the AMT does not hold (`continue` at :249-251): compact their reserved slots away
+    if (any_skip && !ms) {  // receipts the AMT does not hold (`continue` at :249-251): compact their reserved slots away
         ipcfp_event_proof* pp = box->proofs.as<ipcfp_event_proof>();
         uint64_t w = 0;
         for (uint64_t k = 0; k < n_proofs; k++) if (pp[k].exec_index != UINT64_MAX) pp[w++] = pp[k];
         n_proofs = w;
     }
     ipcfp_event_result& r = box->r;
-    r.n_matching = M; r.matching_indices = box->matching.as<uint64_t>();
+    r.n_matching = n_pairs; r.matching_indices = box->matching.as<uint64_t>();
     r.n_proofs = n_proofs; r.proofs = box->proofs.as<ipcfp_event_proof>();
     r.data_blob = box->blob.as<uint8_t>(); r.data_blob_size = n_bytes;
     box->wit.fill(r.witness);
     r.n_exec = n_exec;
-    float ms;
-    IPCFP_CUDA(cudaEventElapsedTime(&ms, s->ev[0], s->ev[5])); r.ms_total = ms;
-    IPCFP_CUDA(cudaEventElapsedTime(&ms, s->ev[1], s->ev[2])); r.ms_txamt = ms;
-    IPCFP_CUDA(cudaEventElapsedTime(&ms, s->ev[2], s->ev[3])); r.ms_pass1 = ms;
-    IPCFP_CUDA(cudaEventElapsedTime(&ms, s->ev[3], s->ev[4])); r.ms_pass2 = ms;
-    IPCFP_CUDA(cudaEventElapsedTime(&ms, s->ev[4], s->ev[5])); r.ms_witness = ms;
+    float el;
+    IPCFP_CUDA(cudaEventElapsedTime(&el, s->ev[0], s->ev[5])); r.ms_total = el;
+    IPCFP_CUDA(cudaEventElapsedTime(&el, s->ev[1], s->ev[2])); r.ms_txamt = el;
+    IPCFP_CUDA(cudaEventElapsedTime(&el, s->ev[2], s->ev[3])); r.ms_pass1 = el;
+    IPCFP_CUDA(cudaEventElapsedTime(&el, s->ev[3], s->ev[4])); r.ms_pass2 = el;
+    IPCFP_CUDA(cudaEventElapsedTime(&el, s->ev[4], s->ev[5])); r.ms_witness = el;
     r.pass1_bytes = pass1_bytes; r.pass1_nodes = pass1_nodes;
     r.shard_raw_total = nraw_total;
     if (sharded) { r.n_exec = 0; r.shard_exec_count = nraw; box->shard_exec = std::move(exec_raw); r.shard_exec_dev = box->shard_exec.p; }

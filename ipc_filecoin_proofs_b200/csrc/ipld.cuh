@@ -348,6 +348,28 @@ __device__ __forceinline__ bool event_matches(const uint8_t* p, const EvLog& ev,
 }
 __device__ __forceinline__ uint32_t topic_offset(const EvLog& ev, uint32_t k) { return ev.case_a ? ev.toff[0] + 32 * k : ev.toff[k]; }
 
+// Up to IPCFP_MAX_EVENT_SPECS EventMatchers tested together (ipcfp_generate_event_proof_multi): bit k of a mask is spec k.
+struct MultiMatcher {
+    Matcher m[IPCFP_MAX_EVENT_SPECS];   // first member: m[0] sits where the single-spec Matcher does
+    uint32_t n;
+};
+// event_matches against every spec at once. The first 8 bytes of topics 0 and 1 are loaded once and screen the specs; a spec that
+// passes the screen is compared in full.
+__device__ __forceinline__ uint64_t event_spec_mask(const uint8_t* p, const EvLog& ev, const MultiMatcher& mm) {
+    if (!ev.some || ev.ntopics < 2) return 0;
+    const uint8_t* p0 = p + ev.toff[0];
+    const uint8_t* p1 = p + (ev.case_a ? ev.toff[0] + 32 : ev.toff[1]);
+    const uint64_t a = load_u64_any(p0), b = load_u64_any(p1);
+    uint64_t mask = 0;
+    for (uint32_t k = 0; k < mm.n; k++) {
+        const Matcher& m = mm.m[k];
+        if (m.t0[0] != a || m.t1[0] != b) continue;
+        if (m.has_actor && ev.emitter != m.actor) continue;
+        if (eq32(p0, m.t0) && eq32(p1, m.t1)) mask |= 1ull << k;
+    }
+    return mask;
+}
+
 // ------------------------------------------------------------------ Receipt = [exit_code, return_data, gas_used, events_root|null]
 __device__ __forceinline__ void parse_receipt(Rd& r) {
     rd_array_exact(r, 4);

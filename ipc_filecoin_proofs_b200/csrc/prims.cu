@@ -114,20 +114,21 @@ template <class Load> __global__ void __launch_bounds__(SCAN_THREADS) k_scan_fin
 
 size_t scan_scratch_elems(uint64_t n) { return (size_t)div_up(n, SCAN_TILE) + 1; }
 
-template <class Load> static void scan_impl(const uint32_t* in, uint64_t* out, uint64_t n, uint64_t* total_dev, uint64_t* scratch, cudaStream_t st, Load load) {
+template <class Load> static void scan_impl(const uint32_t* in, uint64_t* out, uint64_t n, uint64_t* total_dev, uint64_t* scratch, cudaStream_t st, Load load,
+                                            bool fixed_launches) {
     if (n == 0) {
         if (total_dev) IPCFP_CUDA(cudaMemsetAsync(total_dev, 0, 8, st));
         return;
     }
-    if (n <= SCAN_SMALL) { k_scan_small<<<1, SCAN_THREADS, 0, st>>>(in, out, n, total_dev, load); IPCFP_LAUNCH_CHECK(); return; }
+    if (n <= SCAN_SMALL && !fixed_launches) { k_scan_small<<<1, SCAN_THREADS, 0, st>>>(in, out, n, total_dev, load); IPCFP_LAUNCH_CHECK(); return; }
     unsigned nb = div_up(n, SCAN_TILE);
     k_scan_reduce<<<nb, SCAN_THREADS, 0, st>>>(in, n, scratch, load); IPCFP_LAUNCH_CHECK();
     if (nb <= SCAN_FUSED_BLOCKS) { k_scan_final_fused<<<nb, SCAN_THREADS, 0, st>>>(in, out, n, scratch, total_dev, load); IPCFP_LAUNCH_CHECK(); return; }
     k_scan_block_sums<<<1, SCAN_THREADS, 0, st>>>(scratch, nb, total_dev); IPCFP_LAUNCH_CHECK();
     k_scan_final<<<nb, SCAN_THREADS, 0, st>>>(in, out, n, scratch, load); IPCFP_LAUNCH_CHECK();
 }
-void exclusive_scan_u32(const uint32_t* in, uint64_t* out, uint64_t n, uint64_t* total_dev, uint64_t* scratch, cudaStream_t st) {
-    scan_impl(in, out, n, total_dev, scratch, st, LoadIdentity());
+void exclusive_scan_u32(const uint32_t* in, uint64_t* out, uint64_t n, uint64_t* total_dev, uint64_t* scratch, cudaStream_t st, bool fixed_launches) {
+    scan_impl(in, out, n, total_dev, scratch, st, LoadIdentity(), fixed_launches);
 }
 
 // ------------------------------------------------------------------------------------------ bitmap → indices
@@ -143,9 +144,9 @@ __global__ void k_bitmap_scatter(const uint32_t* bits, uint64_t nwords, const ui
     }
 }
 void bitmap_to_indices(const uint32_t* bits, uint64_t nbits, uint32_t* out, uint64_t* total_dev, uint64_t* word_prefix, uint64_t* scratch,
-                       cudaStream_t st) {
+                       cudaStream_t st, bool fixed_launches) {
     uint64_t nwords = (nbits + 31) / 32;
-    scan_impl(bits, word_prefix, nwords, total_dev, scratch, st, LoadPopc());
+    scan_impl(bits, word_prefix, nwords, total_dev, scratch, st, LoadPopc(), fixed_launches);
     if (nwords == 0) return;
     k_bitmap_scatter<<<div_up(nwords, 256), 256, 0, st>>>(bits, nwords, word_prefix, out); IPCFP_LAUNCH_CHECK();
 }
